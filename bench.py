@@ -22,6 +22,8 @@ one read pass (b2s_decompress_*: CRC32C verify + decode + XXH32 verify) over the
   cpu_baseline : the reference's CPU arithmetic (liblz4 / libzstd / restated snappy + framing + XXH32 + CRC32C, oracle/), all
                  host cores the cgroup grants, bounded sample of the same data
 `--impl reference` times that CPU path alone on the same config (the reference itself is Scala on a JVM, absent here).
+`--dump-outputs DIR` writes what the last timed step returned to its caller (rank 0's share) as DIR/<name>.npy, see
+dump_outputs(); the inputs are seeded, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -49,6 +51,46 @@ NCU_TRAFFIC_PER_CODEC_BLOCK = {1: (1.944139e9 + 4.139978e9) / 32768, 4: (1.56430
 METRIC = "shuffle write+read GB/s (compress+CRC) at 1/2/4/8 B200 vs JVM-LZ4 CPU baseline"
 WAVE_BLOCKS_SMALL = 200000   # 65,520-B blocks per resident wave (13.1 GB)
 WAVE_BLOCKS_LARGE = 20000    # 671,112-B blocks per resident wave (13.4 GB)
+# --dump-outputs: the leading bytes of this many shuffle blocks (a seeded choice) are stored as they left the device; the
+# per-block arrays cover every block (<= WAVE_BLOCKS_SMALL of them), so the files stay far below DUMP_LIMIT
+DUMP_SAMPLE_BLOCKS = 16
+DUMP_SAMPLE_BYTES = 256 << 10
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, c, w, r, d_cmp, d_out):
+    """Writes the last timed wave's results as float64 (per-block integers) and float32 (bytes) .npy files:
+    compressed_{offsets,lengths,crc32c,status} from the compress call, decompressed_{offsets,lengths,status} from the
+    decompress call, decompressed_crc32c over every decoded block, and for the blocks in sample_blocks the first
+    DUMP_SAMPLE_BYTES of each compressed stream and of each decoded block, concatenated (compressed_sample,
+    decompressed_sample)."""
+    n = w["dst_len"].size
+    pick = np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_SAMPLE_BLOCKS), replace=False))
+
+    def sample(d_base, offs, lens):
+        parts = []
+        for i in pick:
+            part = np.empty(min(int(lens[i]), DUMP_SAMPLE_BYTES), dtype=np.uint8)
+            if part.size:
+                c.dev_memcpy(part.ctypes.data, d_base + int(offs[i]), part.size, 2)
+            parts.append(part)
+        return np.concatenate(parts).astype(np.float32)
+
+    arrays = {
+        "compressed_offsets": w["dst_off"], "compressed_lengths": w["dst_len"], "compressed_crc32c": w["checksums"],
+        "compressed_status": w["status"], "decompressed_offsets": r["dst_off"], "decompressed_lengths": r["dst_len"],
+        "decompressed_status": r["status"],
+        "decompressed_crc32c": c.checksum_dev(c.CHECKSUM_CRC32C, d_out, r["dst_off"], r["dst_len"]),
+        "sample_blocks": pick,
+    }
+    arrays = {k: np.asarray(v).astype(np.float64) for k, v in arrays.items()}
+    arrays["compressed_sample"] = sample(d_cmp, w["dst_off"], w["dst_len"])
+    arrays["decompressed_sample"] = sample(d_out, r["dst_off"], r["dst_len"])
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, "outputs to dump (%d B) exceed %d B" % (total, DUMP_LIMIT)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def measured_peak():
@@ -230,7 +272,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--codec", default="", choices=["", "lz4", "snappy", "zstd"],
                     help="override the configuration's codec (lz4 = LZ4Block, snappy = xerial, zstd)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.config == 5):
+        ap.error("--dump-outputs needs the device-resident B200 arm (--impl b200, --config 2/3/4)")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -349,7 +395,7 @@ def main():
     t0 = time.perf_counter()
     c.mark(0)                      # CUDA events on the library's own stream (every call is synchronous)
     for _ in range(steps):
-        step_device(True)
+        w, r = step_device(True)
     c.mark(1)
     dev_elapsed = c.marks_elapsed_ms() * 1e-3
     barrier()
@@ -357,6 +403,8 @@ def main():
     elapsed = max_over_ranks(max(dev_elapsed, 0.0) if dev_elapsed > 0.5 * wall else wall)
     clocks = sampler.stop()
     launches = L.b2s_total_kernel_launches() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, c, w, r, d_cmp, d_out)
     ms_per_step = elapsed / steps * 1e3
     value = world * rank_bytes / (elapsed / steps) / 1e9
 

@@ -6,6 +6,7 @@ import re
 import pytest
 
 import spark_s3_shuffle_b200 as pkg
+from without_gpu import rerun_without_gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -54,7 +55,8 @@ def test_fails_loudly_without_a_gpu():
     except Exception:
         has_gpu = os.path.exists("/dev/nvidia0")
     if has_gpu:
-        pytest.skip("GPU present")
+        rerun_without_gpu(__file__, "test_fails_loudly_without_a_gpu")
+        return
     c = pkg.capi
     L = c.load()
     assert L.b2s_init(0, 0, 0) == c.E_CUDA

@@ -13,6 +13,7 @@ import pytest
 
 import spark_s3_shuffle_b200 as pkg
 from shuffle_model import decode_pairs, encode_pairs, oracle_read_partition
+from without_gpu import rerun_without_gpu
 
 host = pkg.host
 
@@ -160,7 +161,8 @@ def test_gpu_mode_fails_loudly_without_a_device(tmp_path):
     try:
         import torch
         if torch.cuda.is_available():
-            pytest.skip("GPU present")
+            rerun_without_gpu(__file__, "test_gpu_mode_fails_loudly_without_a_device")
+            return
     except ImportError:
         pass
     d = host.S3ShuffleDispatcher(new_conf(tmp_path, **{"spark.shuffle.s3.gpu.enabled": True}))
@@ -177,7 +179,8 @@ def test_group_commit_queue_fails_loudly_without_a_device(tmp_path):
     """the queue is plumbing over the C ABI: no GPU, no result (never a CPU path)"""
     import torch
     if torch.cuda.is_available():
-        pytest.skip("needs a box without a GPU")
+        rerun_without_gpu(__file__, "test_group_commit_queue_fails_loudly_without_a_device")
+        return
     d = host.S3ShuffleDispatcher(new_conf(tmp_path))
     with pytest.raises(host.CodecException):
         d.queueCompress(1, [b"abc" * 100], bound=lambda n: n + 64)
